@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the camera->BEV lift (BASELINE.json metric: lift frames/sec, 6-cam 224x480 -> 200x200).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg3_baseline]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg3_baseline] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path {head tensor, intrinsics, extrinsics} -> BEV (B', C, X, Y) over one batch of
 synthetic frames (SURVEY.md section 8d).  Prints ONE JSON line (rank 0).
@@ -39,6 +39,22 @@ from fiery_b200.synthetic import CONFIGS, LiftConfig, make_calibration, make_gra
 
 METRIC = "camera->BEV lift frames/sec (6-cam 224x480 -> 200x200)"
 L2_FLUSH_BYTES = 256 << 20
+DUMP_BYTES = 60 << 20           # --dump-outputs: array data of all files together; with the .npy headers it stays under 64 MB
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """Writes each array as ``out_dir/<name>.npy`` in float32 (float64 stays float64), flattened in logical (C) order when sampled.
+    An array larger than its equal share of DUMP_BYTES is replaced by a sample of its elements at indices drawn from a fixed seed,
+    so two runs with the same arguments store the same elements and two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        a = np.ascontiguousarray(a if a.dtype in (np.float32, np.float64) else a.astype(np.float32))
+        if a.nbytes > share:
+            pick = np.sort(np.random.default_rng(0).choice(a.size, size=share // a.itemsize, replace=False))
+            a = a.reshape(-1)[pick]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def load_traffic(workload: str):
@@ -130,7 +146,7 @@ def _best_thread_count(oracle, head, K, E, candidates):
 def time_cpu_reference(cfg: LiftConfig, frames: int, reps: int, warmup: int = 1, backward: bool = False):
     """Times the oracle's torch-CPU restatement of the reference op chain (fiery.py:193-273, encoder.py:99-100,
     geometry.py:283-314) on the host cores, at the thread count that is fastest on this box.
-    Returns (frames_per_s, seconds_per_call, threads)."""
+    Returns (frames_per_s, seconds_per_call, threads, output of the last timed call)."""
     from oracle import lift_oracle as O
     cores = os.cpu_count() or 1
     sub = LiftConfig(**{**cfg.__dict__, "frames": frames})
@@ -150,10 +166,10 @@ def time_cpu_reference(cfg: LiftConfig, frames: int, reps: int, warmup: int = 1,
     ts = []
     for _ in range(reps):
         t0 = time.perf_counter()
-        cpu_lift_once(oracle, head, K, E, gout)
+        out = cpu_lift_once(oracle, head, K, E, gout)
         ts.append(time.perf_counter() - t0)
     sec = float(np.median(ts))
-    return frames / sec, sec, threads
+    return frames / sec, sec, threads, out
 
 
 def config_dict(cfg: LiftConfig, args, world: int):
@@ -169,9 +185,11 @@ def run_reference(args, cfg: LiftConfig, rank: int):
     if rank != 0:
         return
     frames = cfg.frames                       # the same batch the GPU arm lifts per step
-    steps = max(1, args.steps)
-    fps, sec, threads = time_cpu_reference(cfg, frames, reps=steps, warmup=max(1, min(args.warmup, 2)),
-                                           backward=(args.direction == "fwd_bwd"))
+    steps = args.steps
+    backward = args.direction == "fwd_bwd"
+    fps, sec, threads, out = time_cpu_reference(cfg, frames, reps=steps, warmup=max(1, min(args.warmup, 2)), backward=backward)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"grad_head" if backward else "bev": out})
     line = {
         "impl": "reference", "metric": METRIC, "value": fps, "unit": "frames/s", "n_gpus": args.gpus, "steps": steps,
         "warmup": args.warmup, "ms_per_step": sec * 1e3, "higher_is_better": True, "scaling": "weak",
@@ -214,7 +232,7 @@ def run_train(args, cfg: LiftConfig, rank: int, local_rank: int, world: int):
     batch = synthetic_batch(cfg, b, s, dev, seed=1000, feature_input=True, first_sample=rank * b)
     host = {k: v.cpu().pin_memory() for k, v in batch.items()}
     flush = torch.empty(L2_FLUSH_BYTES // 4, dtype=torch.float32, device=dev)
-    W, S = max(args.warmup, 3), max(args.steps, 1)
+    W, S = max(args.warmup, 3), args.steps
 
     def barrier():
         if distributed:
@@ -231,8 +249,10 @@ def run_train(args, cfg: LiftConfig, rank: int, local_rank: int, world: int):
         torch.cuda.synchronize()
         return float(np.mean([a.elapsed_time(e) for a, e in pairs]))
 
+    last = {}
+
     def step_dev():
-        trainer.step(batch)
+        last["loss"] = trainer.step(batch)
 
     def step_e2e():                                   # the step's inputs come from pinned host memory, its loss goes back to the host
         dev_batch = {k: v.to(dev, non_blocking=True) for k, v in host.items()}
@@ -247,6 +267,9 @@ def run_train(args, cfg: LiftConfig, rank: int, local_rank: int, world: int):
         step_dev()
     barrier()
     ms_dev = timed(step_dev)
+    if args.dump_outputs and rank == 0:               # the last timed step's loss and the weights its optimizer step left
+        dump_outputs(args.dump_outputs, {"loss": last["loss"],
+                                         "params": torch.cat([p.detach().flatten() for p in trainer.bucket.params])})
     barrier()
     for _ in range(2):
         step_e2e()
@@ -305,7 +328,7 @@ def run_train(args, cfg: LiftConfig, rank: int, local_rank: int, world: int):
             "clocks": clocks,
         }
         if not args.no_cpu_baseline:
-            fps, sec, threads = time_cpu_reference(cfg, min(frames, args.cpu_frames), reps=max(2, args.cpu_reps // 2), backward=True)
+            fps, sec, threads, _ = time_cpu_reference(cfg, min(frames, args.cpu_frames), reps=max(2, args.cpu_reps // 2), backward=True)
             line["cpu_baseline"] = {"value": fps, "unit": "frames/s", "cores": threads, "kind": "port",
                                     "sample": f"forward+backward of the lift (oracle/lift_oracle.py through torch autograd) on "
                                               f"{min(frames, args.cpu_frames)} frame(s) of {cfg.name}, {threads} threads"}
@@ -337,7 +360,13 @@ def main():
                                                       "sizes of the first stages (the last repeats)")
     ap.add_argument("--cpu-frames", type=int, default=3)
     ap.add_argument("--cpu-reps", type=int, default=5)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed path returned in its last step as DIR/<name>.npy (rank 0; "
+                         "float32, at most 64 MB in all: a larger output is replaced by a fixed seeded sample of its elements). "
+                         "forward: bev; fwd_bwd: loss and the updated params; --impl reference: bev, or grad_head with fwd_bwd")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = CONFIGS[args.workload]
 
     rank = int(os.environ.get("RANK", "0"))
@@ -380,7 +409,7 @@ def main():
     if head_dtype != torch.float32:
         head_d = head_d.to(head_dtype)
     flush = torch.empty(L2_FLUSH_BYTES // 4, dtype=torch.float32, device=dev)
-    W, S = max(args.warmup, 3), max(args.steps, 1)
+    W, S = max(args.warmup, 3), args.steps
     X, Y = cfg.bev_hw
 
     def barrier():
@@ -429,6 +458,8 @@ def main():
         step_eager()
     barrier()
     t_dev = timed_steps(graphed, S)
+    if args.dump_outputs and rank == 0:               # the BEV of the last timed replay, before anything replays the graph again
+        dump_outputs(args.dump_outputs, {"bev": graphed.output})
     barrier()
     t_dev_noflush = timed_steps(graphed, S, do_flush=False)
     t_static = timed_steps(graphed_static, S)
@@ -822,7 +853,7 @@ def main():
                                                 "ms_per_step": float(np.mean(t_ref_gpu)),
                                                 "what": "oracle/lift_oracle.py (the reference's PyTorch op chain) on CUDA tensors, "
                                                         "torch library kernels, same inputs, 5 steps"}
-            fps, sec, threads = time_cpu_reference(cfg, min(frames, args.cpu_frames), reps=args.cpu_reps)
+            fps, sec, threads, _ = time_cpu_reference(cfg, min(frames, args.cpu_frames), reps=args.cpu_reps)
             line["cpu_baseline"] = {"value": fps, "unit": "frames/s", "cores": threads, "kind": "port",
                                     "sample": f"{args.cpu_reps} reps of {min(frames, args.cpu_frames)} frame(s) of {cfg.name}: "
                                               f"torch-CPU op chain of the reference (oracle/lift_oracle.py), median, "

@@ -6,9 +6,18 @@ import pytest
 import torch
 
 from oracle import lift_oracle as O
-from tests._cases import GOLDEN_CASES, build_case, case_id, golden_str, golden_tag, sha
+from tests._cases import GOLDEN_CASES, GOLDEN_THREADS, build_case, case_id, golden_str, golden_tag, sha
 
 FAST_CASES = [c for c in GOLDEN_CASES if c[0] in ("cfg1_tiny", "cfg2_static_lss")]
+
+
+@pytest.fixture(autouse=True, scope="module")
+def recorded_thread_count():
+    """The oracle's CPU ops run with the thread count the golden vectors were recorded with, whatever the host's core count."""
+    before = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(before)
 
 
 @pytest.mark.parametrize("name", ["singletons", "one_voxel", "long_runs", "first_last_boundaries", "random_runs",
